@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the sonar front end (BASELINE.json metric: sonar frames/sec, CFAR + ICP).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--frames F] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--frames F] [--impl ours|reference] [--dump-outputs DIR]
 
 Workload (BASELINE config 4, the configuration the metric is quoted on): a synthetic bag replay --
 F = 4096 polar sonar frames (512 beams x 512 range bins, uint8) per step and per GPU, rendered from a
@@ -65,6 +65,8 @@ def parse():
     ap.add_argument("--pairs", type=int, default=80000, help="config 5: size of the scan-match backlog (0: skip)")
     ap.add_argument("--pair-steps", type=int, default=2, help="config 5: timed steps (after one warm-up step)")
     ap.add_argument("--pair-chunks", type=int, default=8, help="config 5: pieces per shard in the pipelined scatter")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step computed (rank 0) as DIR/<name>.npy, to compare two builds")
     return ap.parse_args()
 
 
@@ -295,6 +297,36 @@ def run_reference(args):
 
 
 # ------------------------------------------------------------------------------------ GPU side
+DUMP_FRAMES = 4096   # --dump-outputs: per-frame results of at most this many frames (a seeded sample of larger steps)
+DUMP_CLOUDS = 256    # and the filtered clouds of at most this many of them (<= 256 x cap_points x 8 B = 16 MiB)
+
+
+def last_step_outputs(ctx, fe, F):
+    """What the last sfe_frontend_run_dev call left on the device, read as its caller reads it
+    (sfe_frontend_results_dev): for a fixed seeded sample of the F frames (all of them up to DUMP_FRAMES) the scan-match
+    result T, iterations, inliers, status and the size of the filtered cloud, and the clouds themselves (x, y rows,
+    concatenated in frame order) of a seeded sub-sample.  Integer outputs are stored as float64 (exact)."""
+    r = fe.results_dev()
+    rng = np.random.default_rng(0)
+    frames = np.sort(rng.choice(F, min(F, DUMP_FRAMES), replace=False))
+    cloud_frames = np.sort(rng.choice(frames, min(len(frames), DUMP_CLOUDS), replace=False))
+    out = {"frame_index": frames.astype(np.float64), "T": ctx.to_host(r["T"], (F, 3, 3), np.float32)[frames]}
+    for k in ("iterations", "inliers", "status", "cloud_count"):
+        out[k] = ctx.to_host(r[k], (F,), np.int32)[frames].astype(np.float64)
+    stride, count = r["cloud_stride"], ctx.to_host(r["cloud_count"], (F,), np.int32)
+    clouds = [ctx.to_host(r["cloud_xy"] + int(f) * stride * 8, (min(int(count[f]), stride), 2), np.float32)
+              for f in cloud_frames]
+    out["cloud_frame_index"] = cloud_frames.astype(np.float64)
+    out["cloud_xy"] = np.concatenate(clouds) if clouds else np.zeros((0, 2), np.float32)
+    return out
+
+
+def dump_outputs(directory, arrays):
+    os.makedirs(directory, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(directory, name + ".npy"), a)
+
+
 def make_pair_backlog(P, device, n_scenes=32, ns=2000, nt=20000):
     """Config 3 / 5 input on `device`: P (source, target, guess) records tiled from `n_scenes` seeded scenes of
     synth.make_icp_pair (SURVEY 8(d) config 3: 2 000-point scan vs 20 000-point submap, identity guess).  The solver
@@ -408,6 +440,8 @@ def run_ours(args):
     barrier()
     dev_ms = max_over_ranks(e0.elapsed_time(e1))
     launches = ctx.launches - l0
+    # read now: the legs below run on the same handle and overwrite the results
+    outputs = last_step_outputs(ctx, fe, F) if args.dump_outputs and rank == 0 else None
 
     # ---- end-to-end leg: host buffers in, results out, through one C-ABI call per step
     for _ in range(W):
@@ -587,6 +621,8 @@ def run_ours(args):
                                                   "filters and ICP (oracle/)"}
             except Exception as e:  # noqa: BLE001
                 line["cpu_baseline"] = {"error": str(e)}
+        if outputs is not None:
+            dump_outputs(args.dump_outputs, outputs)
         print(json.dumps(line), flush=True)
     if world > 1:
         sys.stdout.flush()

@@ -1,7 +1,12 @@
 """CPU-only: the CPU legs of bench.py (cpu_baseline / --impl reference) run and speak the JSON contract."""
 import json
+import os
 import subprocess
 import sys
+
+import numpy as np
+
+BENCH = os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "bench.py")
 
 
 def test_cpu_pipeline_leg_runs_on_a_tiny_sample():
@@ -41,8 +46,68 @@ def test_bench_refuses_to_run_the_product_path_without_a_gpu():
     import torch
     if torch.cuda.is_available():
         return
-    r = subprocess.run([sys.executable, "bench.py", "--steps", "1", "--warmup", "0"], capture_output=True, text=True)
+    r = subprocess.run([sys.executable, BENCH, "--steps", "1", "--warmup", "0"], capture_output=True, text=True)
     assert r.returncode != 0 and "no CUDA device" in (r.stderr + r.stdout)
+
+
+class _FakeDevice:
+    """Stands in for the library context and front end: device memory is one host byte buffer, addresses are offsets
+    into it (starting at 4096 so that no buffer sits at address 0)."""
+
+    def __init__(self, F, stride, rng):
+        self.mem = bytearray(4096)
+        self.F, self.stride = F, stride
+        self.T = rng.normal(size=(F, 3, 3)).astype(np.float32)
+        self.ints = {k: rng.integers(0, 50, F).astype(np.int32) for k in ("iterations", "inliers", "status")}
+        self.count = rng.integers(0, stride + 3, F).astype(np.int32)   # a few above the stride: truncated clouds
+        self.xy = rng.normal(size=(F, stride, 2)).astype(np.float32)
+        self.addr = {k: self._put(a) for k, a in
+                     dict(T=self.T, cloud_count=self.count, cloud_xy=self.xy, **self.ints).items()}
+
+    def _put(self, a):
+        at = len(self.mem)
+        self.mem += a.tobytes()
+        return at
+
+    def to_host(self, ptr, shape, dtype):
+        n = int(np.prod(shape)) * np.dtype(dtype).itemsize
+        return np.frombuffer(bytes(self.mem[ptr:ptr + n]), dtype).reshape(shape).copy()
+
+    def results_dev(self):
+        return dict(self.addr, cloud_stride=self.stride)
+
+
+def test_dumped_outputs_sample_and_bound(tmp_path):
+    """bench.py --dump-outputs: a step of up to DUMP_FRAMES frames is kept whole; a larger one is sampled with a fixed
+    seed (the same frames every run); clouds are read at the library's stride and clipped to it; every file is
+    float32 or float64 and the total stays under 64 MiB even for the largest clouds."""
+    import bench
+    rng = np.random.default_rng(3)
+    small = _FakeDevice(40, 16, rng)
+    out = bench.last_step_outputs(small, small, small.F)
+    assert np.array_equal(out["frame_index"], np.arange(small.F)) and np.array_equal(out["T"], small.T)
+    for k, v in small.ints.items():
+        assert np.array_equal(out[k], v) and out[k].dtype == np.float64
+    assert np.array_equal(out["cloud_count"], small.count)
+    want = np.concatenate([small.xy[f, :min(small.count[f], small.stride)] for f in range(small.F)])
+    assert np.array_equal(out["cloud_frame_index"], np.arange(small.F)) and np.array_equal(out["cloud_xy"], want)
+
+    big = _FakeDevice(bench.DUMP_FRAMES + 500, 4, rng)
+    a, b = bench.last_step_outputs(big, big, big.F), bench.last_step_outputs(big, big, big.F)
+    assert all(np.array_equal(a[k], b[k]) for k in a)
+    idx = a["frame_index"].astype(int)
+    assert len(idx) == bench.DUMP_FRAMES and np.all(np.diff(idx) > 0) and idx[-1] < big.F
+    assert np.array_equal(a["T"], big.T[idx]) and np.array_equal(a["status"], big.ints["status"][idx])
+    cf = a["cloud_frame_index"].astype(int)
+    assert len(cf) == bench.DUMP_CLOUDS and np.isin(cf, idx).all()
+    assert np.array_equal(a["cloud_xy"], np.concatenate([big.xy[f, :min(big.count[f], big.stride)] for f in cf]))
+
+    bench.dump_outputs(str(tmp_path / "d"), a)
+    for k in a:
+        assert np.load(tmp_path / "d" / f"{k}.npy").dtype in (np.float32, np.float64), k
+    cap_points = 8192    # sfe_frontend_params_default
+    worst = bench.DUMP_FRAMES * (9 * 4 + 5 * 8) + bench.DUMP_CLOUDS * (cap_points * 2 * 4 + 8)
+    assert worst < 64 * 2**20
 
 
 def test_clock_sampler_keeps_the_load_until_samples_arrive(tmp_path, monkeypatch):

@@ -11,8 +11,8 @@ what an unpinned stage can offer):
     the worst of 200 scans, 1e-5 m on the median one.
 
 200 BASELINE-config-3 pairs (2 000 x 20 000 points, identity guess) x {fixed 20 iterations, shipped checkers} and
-200 pipeline-sized problems (~350 x ~1 100 points, odometry-like guesses).  The deviation histograms are printed and
-written to gpurun_out/icp_parity_sweep.json (copied to profiles/ by the round's evidence pass)."""
+200 pipeline-sized problems (~350 x ~1 100 points, odometry-like guesses).  The deviation histograms are printed and,
+when SFE_ICP_SWEEP_REPORT names a file, written there as JSON (profiles/r02_icp_parity_sweep.json is one)."""
 import json
 import os
 
@@ -129,9 +129,9 @@ def _sweep(name, pairs, guesses, kw, fixed_iters):
 def sweep_log():
     log = {}
     yield log
-    os.makedirs("gpurun_out", exist_ok=True)
-    with open("gpurun_out/icp_parity_sweep.json", "w") as f:
-        json.dump(log, f, indent=1)
+    if os.environ.get("SFE_ICP_SWEEP_REPORT"):
+        with open(os.environ["SFE_ICP_SWEEP_REPORT"], "w") as f:
+            json.dump(log, f, indent=1)
 
 
 @pytest.mark.parametrize("mode", ["fixed20", "checkers"])

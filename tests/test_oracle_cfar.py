@@ -1,7 +1,7 @@
 """CPU-only: pin the CFAR oracle (oracle/cfar_ref.c) against the reference.
 
- * against oracle/_ref/libcfar_ref.so = the UNMODIFIED reference cfar.cpp compiled from
-   /root/reference (present in the dev container and, as a prebuilt file, on the GPU box);
+ * against tests/golden/cfar_reference.npz, what the UNMODIFIED reference cfar.cpp
+   (oracle/_ref/libcfar_ref.so) returned on the inputs below (tools/make_golden.py);
  * against tests/golden/cfar_masks.npz, produced by running the reference's own CFAR class
    (tools/make_golden.py).
 """
@@ -26,17 +26,24 @@ def _inputs():
     yield "negative_and_big", (rng.normal(0, 1e6, (80, 17))).astype(np.float32), 6, 1, 11
 
 
-@pytest.mark.skipif(not orc.have_reference(), reason="oracle/_ref not built (needs /root/reference once)")
+def _sha256(a):
+    return hashlib.sha256(np.ascontiguousarray(a).tobytes()).hexdigest()
+
+
 @pytest.mark.parametrize("alg", ALGS)
-def test_port_equals_unmodified_reference(alg):
+def test_port_equals_unmodified_reference(alg, golden_dir):
+    g = np.load(f"{golden_dir}/cfar_reference.npz")
     for name, img, T, G, k in _inputs():
-        for tau in (TAU[alg], 0.37):
-            m0, t0 = orc.cfar_reference(alg, img, T, G, k, tau, want_thr=True)
+        assert _sha256(img) == str(g[name + "_input_sha256"]), name  # the inputs the fixture was made from
+        for i, tau in enumerate((TAU[alg], 0.37)):
+            key = f"{name}_{alg}_{i}"
             m1, t1 = orc.cfar(alg, img, T, G, k, tau, want_thr=True)
-            assert np.array_equal(m0, m1), (name, alg)
-            assert np.array_equal(t0.view(np.uint32), t1.view(np.uint32)), (name, alg)  # bit-exact thresholds
-            m2, _ = orc.cfar_reference(alg, img, T, G, k, tau, want_thr=False)
-            assert np.array_equal(m0, m2)
+            assert np.array_equal(np.packbits(np.ascontiguousarray(m1)), g[key + "_mask"]), key
+            t1 = np.ascontiguousarray(t1)
+            assert np.array_equal(t1[::7, ::5].view(np.uint32), g[key + "_thr_sample"].view(np.uint32)), key
+            assert _sha256(t1) == str(g[key + "_thr_sha256"]), key  # bit-exact thresholds
+            m2, _ = orc.cfar(alg, img, T, G, k, tau, want_thr=False)
+            assert np.array_equal(m1, m2), key
 
 
 @pytest.mark.parametrize("alg", ALGS)

@@ -32,6 +32,8 @@ Fixtures written:
                                     target grid (packed) and the cost of 96 candidate poses.
                                     gtsam is absent: gtsam.Pose2 is replaced by the SE(2) class
                                     of oracle/globalinit_ref.py, everything else is the reference
+  tests/golden/cfar_reference.npz   the unmodified cfar.cpp on the inputs of
+                                    tests/test_oracle_cfar.py (masks, threshold digests + samples)
 """
 import hashlib
 import importlib
@@ -350,9 +352,39 @@ def fov_fixture():
     print("fov_select:", len(target_points), "targets ->", int(ns["sel"].sum()), "kept; written to", out)
 
 
+def cfar_reference_fixture():
+    """tests/golden/cfar_reference.npz: the unmodified reference cfar.cpp (oracle/_ref/libcfar_ref.so) on the inputs
+    of tests/test_oracle_cfar.py, every algorithm, two threshold factors.  Masks are stored packed; threshold images by
+    the SHA-256 of their bytes (bit-exact) and a strided sample.  Needs the reference tree to build oracle/_ref."""
+    from oracle import oracle as orc
+    sys.path.insert(0, os.path.join(REPO, "tests"))
+    from test_oracle_cfar import ALGS, TAU, _inputs
+    orc.build()
+    assert orc.have_reference(), "oracle/_ref/libcfar_ref.so was not built (reference tree absent)"
+    g = {}
+    for name, img, T, G, k in _inputs():
+        g[name + "_input_sha256"] = np.array(_digest(img))
+        for alg in ALGS:
+            for i, tau in enumerate((TAU[alg], 0.37)):
+                m, thr = orc.cfar_reference(alg, img, T, G, k, tau, want_thr=True)
+                m_only, _ = orc.cfar_reference(alg, img, T, G, k, tau, want_thr=False)
+                assert np.array_equal(m, m_only), (name, alg, i)
+                thr = np.ascontiguousarray(thr)
+                key = f"{name}_{alg}_{i}"
+                g[key + "_mask"] = np.packbits(np.ascontiguousarray(m))
+                g[key + "_thr_sha256"] = np.array(_digest(thr))
+                g[key + "_thr_sample"] = thr[::7, ::5].copy()
+    out = os.path.join(REPO, "tests", "golden", "cfar_reference.npz")
+    np.savez_compressed(out, **g)
+    print("cfar_reference:", len(g), "arrays written to", out)
+
+
 if __name__ == "__main__":
     if "--only-fov" in sys.argv:
         fov_fixture()
+    elif "--only-cfar-reference" in sys.argv:
+        cfar_reference_fixture()
     else:
         main()
         fov_fixture()
+        cfar_reference_fixture()
